@@ -38,6 +38,7 @@ WORKLOAD = ("synthetic 1080p@25fps: batched CNN detect (upsample 1, every frame)
             "(%d live tracks x fwd+bwd) + %d faces/frame 68-pt landmarks + ResNet-v1 embed"
             % (2 * TRACKS_PER_STREAM, TRACKS_PER_STREAM, FACES_PER_FRAME))
 TRACKER_BYTES_PER_UPDATE = 2.07e6      # SURVEY.md §8(d): A read + written (f32 complex 31x64x64), B, chip
+DUMP_MAX_BYTES = 64 << 20
 
 
 def time_index(s):
@@ -88,6 +89,21 @@ class ClockSampler(threading.Thread):
                 reasons.append(nme)
         return dict(sm_mhz=(sm[len(sm) // 2] if sm else None), sm_max_mhz=(max(mx) if mx else None), reasons=reasons,
                     samples=len(self.rows))
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """--dump-outputs: `arrays` (name -> numpy array) as out_dir/<name>.npy, float64 kept, everything else as float32
+    (integer outputs are small coordinates and counts, exact in float32).  Above DUMP_MAX_BYTES in all, every array keeps
+    the same seeded sample of its leading-axis rows, so two runs with the same arguments write the same rows."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(a, np.float64 if a.dtype == np.float64 else np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_MAX_BYTES and a.shape[0] > 1:
+            keep = max(1, a.shape[0] * DUMP_MAX_BYTES // total)
+            a = a[np.sort(np.random.default_rng(seed).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_models():
@@ -217,7 +233,12 @@ def main():
     ap.add_argument("--ncu-step", action="store_true",
                     help="after the warm-up, run ONE serialised step between cudaProfilerStart/Stop and exit (for `ncu "
                          "--profile-from-start off`: the launch list / --set full capture of exactly one step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (detections, landmarks, embeddings, "
+                         "tracker state; rank 0) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -409,6 +430,15 @@ def main():
         sys.stderr.write("[bench debug] tracker state after the resident leg: |coord| max %.4g, width %.4g..%.4g, psr %.4g..%.4g, finite %s\n"
                          % (float(st_[:, :4].abs().max()), float(wd_.min()), float(wd_.max()), float(st_[:, 4].min()),
                             float(st_[:, 4].max()), bool(torch.isfinite(st_).all())))
+    if args.dump_outputs and rank == 0:
+        # the detector's boxes / scores are padded to MAX_DET per frame; slots past a frame's count hold stale data
+        kept = torch.arange(det0.MAX_DET, device=dev)[None, :] < res["det_counts"].clamp(max=det0.MAX_DET)[:, None]
+        outs = dict(det_boxes=torch.where(kept[..., None], res["det_boxes"], 0),
+                    det_scores=torch.where(kept, res["det_scores"], 0.0),
+                    det_counts=res["det_counts"], landmarks=res["landmarks"], embeddings=res["embeddings"])
+        if use_tracker:
+            outs["tracker_state"] = bank.read_state(trk_ids)
+        dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in outs.items()})
 
     # ---------------- end-to-end timing (host buffers, H2D + D2H inside) ----------------
     run_e2e(min(max(args.warmup, 1), 2))
