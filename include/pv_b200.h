@@ -430,6 +430,46 @@ int pv_tracker_update_frames(void* handle, const void* frames, int H, int W, con
 /* device pointers owned by the bank: positions f32 [capacity,4] and PSR f32 [capacity] */
 int pv_tracker_state(void* handle, float** pos, float** psr);
 
+/* ------------------------------------------------------------------------------------------
+ * shot boundary detection (csrc/shot.cu) — pyannote/video/structure/shot.py: gray + resize, Farneback optical
+ * flow (pyr_scale 0.5, 3 levels, winsize 15, 3 iterations, poly_n 5, poly_sigma 1.1, box-filter update) and the
+ * displaced frame difference of every consecutive pair.  Geometry and tables are built by pyannote_video_b200/shot.py.
+ * ------------------------------------------------------------------------------------------ */
+#define PV_SHOT_MAX_LEVELS 4
+#define PV_SHOT_MAX_TAPS 19
+#define PV_SHOT_POLY_N 5
+#define PV_SHOT_WINSIZE 15
+#define PV_SHOT_ITERATIONS 3
+typedef struct PvShotLevel {
+  int32_t rows, cols;
+  int32_t r_off;            /* float offset of the level's R [5, rows, cols] in a frame's R block            */
+  int32_t radius;           /* pre-blur radius (taps = 2 * radius + 1), reflect-101 border                     */
+  int32_t area2x;           /* 1: the level is an exact 2x downscale of level 0 (2x2 mean)                    */
+  int32_t dn_off;           /* float offset in tab of the level-0 -> level resize table (-1: none)             */
+  int32_t up_off;           /* float offset in tab of the coarser-level -> level flow resize table (-1: none)  */
+  float taps[PV_SHOT_MAX_TAPS];
+} PvShotLevel;
+typedef struct PvShotGeo {
+  int32_t h, w;             /* level-0 gray frame: rows, columns                                               */
+  int32_t n_levels;         /* lv[0] is the coarsest level, lv[n_levels - 1] is level 0                        */
+  int32_t r_stride;         /* floats of one frame's R block (all levels)                                      */
+  PvShotLevel lv[PV_SHOT_MAX_LEVELS];
+  float pg[2 * PV_SHOT_POLY_N + 1], pxg[2 * PV_SHOT_POLY_N + 1], pxxg[2 * PV_SHOT_POLY_N + 1];
+  int32_t pad_;
+  double ig11, ig03, ig33, ig55;
+} PvShotGeo;
+/* RGB u8 [B,H,W,3] -> gray u8 [B,h,w]; tab: device int32 x0 x1 cx0 cx1 [w] then y0 y1 cy0 cy1 [h] (11-bit weights) */
+int pv_shot_gray_resize(const void* rgb, int B, int H, int W, const int* tab, int h, int w, void* out, void* stream);
+/* global workspace floats per CTA when the shared-memory budget is exceeded (-1: bad geometry) */
+int64_t pv_shot_polyexp_work_floats(const PvShotGeo* geo);
+int64_t pv_shot_flow_work_floats(const PvShotGeo* geo);
+/* gray u8 [B,h,w] -> R f32 [B, r_stride]; work: B * n_levels * polyexp_work_floats floats, or NULL if it fits on chip */
+int pv_shot_polyexp(const void* gray, int B, const PvShotGeo* geo, const float* tab, float* work, float* R, void* stream);
+/* pairs (p, p+1), p < P, of gray u8 [P+1,h,w] and R [P+1, r_stride] -> dfd f64 [P]; flow_out f32 [P,h,w,2] or NULL;
+ * work: P * flow_work_floats floats, or NULL if it fits on chip */
+int pv_shot_flow_dfd(const void* gray, const float* R, int P, const PvShotGeo* geo, const float* tab, float* work,
+                     double* dfd, float* flow_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -16,6 +16,7 @@ _EXPORTS = {
     "DRect": ("geometry", "DRect"),
     "Point": ("geometry", "Point"),
     "FullObjectDetection": ("geometry", "FullObjectDetection"),
+    "Shot": ("shot", "Shot"),
 }
 
 __all__ = sorted(_EXPORTS)

@@ -8,6 +8,8 @@ Mirrors `scripts/pyannote-face.py` of the reference (usage string at :29-89; `tr
   pyannote-face-b200 detect  [options] <video> <detections>        (new: raw per-frame detections)
   pyannote-face-b200 embed   ...                                     (alias of extract)
   pyannote-face-b200 cluster [--threshold=0.6] <embeddings> <labels> (notebook cells 18-22 as a verb)
+  pyannote-face-b200 shot    [--height=50] [--window=2.0] [--threshold=1.0] <video> <output.json>
+                             (pyannote-structure.py shot: the <shot.json> that `track` reads)
 
 `docopt`, `ffmpeg` and `pyannote.core` do not exist in the build environment, hence argparse and a
 frame source that reads `.npy` arrays ([T,H,W,3] uint8) or `synthetic:<W>x<H>:<frames>[:<seed>]`;
@@ -48,6 +50,23 @@ class ArrayVideo(object):
     @property
     def frame_size(self):
         return self._frame_size
+
+    # the attributes pyannote.video.Video exposes to Shot: frame size (width, height), frame step, time range
+    @property
+    def _size(self):
+        return self._frame_size
+
+    @property
+    def step(self):
+        return 1.0 / self.frame_rate
+
+    @property
+    def start(self):
+        return 0.0
+
+    @property
+    def end(self):
+        return self.duration
 
     @frame_size.setter
     def frame_size(self, value):
@@ -194,6 +213,20 @@ def detect(video, output, face=None, detector=None):
                                                                           r=r.right() / w, b=r.bottom() / h))
 
 
+def shot_cmd(video, output, height=50, window=2.0, threshold=1.0):
+    """Shot boundaries as a pyannote.core Timeline JSON, the file `track` reads"""
+    from .shot import Shot
+    return write_timeline(Shot(video, height=height, context=window, threshold=threshold), output)
+
+
+def write_timeline(segments, output):
+    """segments -> {"pyannote": "Timeline", "content": [{"start", "end"}, ...]} (pyannote.core's JSON)"""
+    content = [{"start": float(s.start), "end": float(s.end)} for s in segments]
+    with open(output, "w") as f:
+        json.dump({"pyannote": "Timeline", "content": content}, f)
+    return content
+
+
 def cluster_cmd(embeddings, output, threshold=0.6, metric="euclidean"):
     from .clustering import FaceClustering
     clustering = FaceClustering(threshold=threshold, metric=metric)
@@ -245,6 +278,12 @@ def main(argv=None):
     p.add_argument("labels")
     p.add_argument("--threshold", type=float, default=0.6)
     p.add_argument("--metric", default="euclidean", choices=["euclidean", "cosine"])
+    p = sub.add_parser("shot")
+    p.add_argument("video")
+    p.add_argument("output")
+    p.add_argument("--height", type=int, default=50)
+    p.add_argument("--window", type=float, default=2.0)
+    p.add_argument("--threshold", type=float, default=1.0)
     a = ap.parse_args(argv)
     if a.verb == "track":
         track(open_video(a.video, a.frame_rate), a.shot, a.tracking, detect_min_size=a.min_size, detect_every=a.every,
@@ -255,6 +294,8 @@ def main(argv=None):
                 a.embeddings, reference_quirks=a.reference_quirks)
     elif a.verb == "detect":
         detect(open_video(a.video, a.frame_rate), a.detections, detector=a.detector)
+    elif a.verb == "shot":
+        shot_cmd(open_video(a.video, a.frame_rate), a.output, height=a.height, window=a.window, threshold=a.threshold)
     elif a.verb == "cluster":
         cluster_cmd(a.embeddings, a.labels, threshold=a.threshold, metric=a.metric)
     return 0
