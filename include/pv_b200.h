@@ -470,6 +470,37 @@ int pv_shot_polyexp(const void* gray, int B, const PvShotGeo* geo, const float* 
 int pv_shot_flow_dfd(const void* gray, const float* R, int P, const PvShotGeo* geo, const float* tab, float* work,
                      double* dfd, float* flow_out, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * shot threading (csrc/orb.cu) — pyannote/video/structure/thread.py: RGB resize then gray, cv2.ORB_create() features
+ * (500 features, scale 1.2, 8 levels, edge 31, FAST 20, Harris, patch 31, WTA_K 2) and the exact Hamming 2-NN
+ * ratio count (best < 0.7 * second, float64) of shot pairs.  Geometry and tables are built by
+ * pyannote_video_b200/thread.py.
+ * ------------------------------------------------------------------------------------------ */
+#define PV_ORB_LEVELS 8
+typedef struct PvOrbGeo {
+  int32_t n_levels;
+  int32_t rows[PV_ORB_LEVELS], cols[PV_ORB_LEVELS];
+  int32_t off[PV_ORB_LEVELS];      /* byte offset of level k in a frame's pyramid plane                             */
+  int32_t tab_off[PV_ORB_LEVELS];  /* int offset in tab of level k's INTER_LINEAR_EXACT taps from level k - 1:
+                                      x offset [cols], x weight [cols], y offset [rows], y weight [rows] (k >= 1)  */
+  int32_t quota[PV_ORB_LEVELS];    /* features kept per level (ties at the cut are all kept)                       */
+  float scale[PV_ORB_LEVELS];      /* keypoint coordinate scale of level k (float32 1.2^k)                         */
+  float gauss[7];                  /* the 7-tap sigma-2 float32 Gaussian of the descriptor smoothing               */
+  int32_t plane;                   /* bytes of one frame's pyramid plane (sum of rows * cols)                      */
+  int32_t cand_cap;                /* keypoint slots per frame: bounds the non-max-suppression survivors           */
+} PvOrbGeo;
+/* RGB u8 [B,H,W,3] -> per channel INTER_LINEAR resize, then RGB2GRAY -> u8 [B,h,w]; tab as pv_shot_gray_resize */
+int pv_orb_resize_gray(const void* rgb, int B, int H, int W, const int* tab, int h, int w, void* gray, void* stream);
+/* workspace bytes per frame of pv_orb_detect (-1: bad geometry) */
+int64_t pv_orb_work_bytes(const PvOrbGeo* geo);
+/* gray u8 [B,h,w] -> per frame f: count[f] keypoints (-1: candidate overflow) in kp f32 [B, cand_cap, 5]
+ * (x, y, octave, response, angle; sorted by octave, y, x) and desc u8 [B, cand_cap, 32]; work: B * work_bytes */
+int pv_orb_detect(const void* gray, int B, const PvOrbGeo* geo, const int* tab, void* work, float* kp, void* desc,
+                  int* count, void* stream);
+/* desc u8 [N,32] packed by frame (offsets i32 [F+1]); pairs i32 [P,2] (query frame, train frame) -> counts i32 [P]:
+ * queries whose best Hamming distance < 0.7 * the second best; 0 when either side has < 2 descriptors */
+int pv_thread_match(const void* desc, const int* offsets, const int* pairs, int P, int* counts, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -17,6 +17,7 @@ _EXPORTS = {
     "Point": ("geometry", "Point"),
     "FullObjectDetection": ("geometry", "FullObjectDetection"),
     "Shot": ("shot", "Shot"),
+    "Thread": ("thread", "Thread"),
 }
 
 __all__ = sorted(_EXPORTS)

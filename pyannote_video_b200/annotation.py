@@ -4,7 +4,25 @@
 `Annotation` objects (pyannote/video/face/clustering.py:59-82,138-148; notebook cells 18-22 iterate them with
 `itertracks(yield_label=True)`).  Only the part of the interface that path uses is provided.
 """
+import itertools
+import string
 from collections import namedtuple
+
+DEFAULT_TRACK = "_"
+
+
+def string_generator():
+    """A, B, ..., Z, AA, AB, ... (pyannote.core.utils.generators.string_generator)"""
+    for n in itertools.count(1):
+        for letters in itertools.product(string.ascii_uppercase, repeat=n):
+            yield "".join(letters)
+
+
+def pairwise(iterable):
+    """(s0, s1), (s1, s2), ..."""
+    a, b = itertools.tee(iterable)
+    next(b, None)
+    return zip(a, b)
 
 
 class Segment(namedtuple("Segment", ["start", "end"])):
@@ -32,8 +50,15 @@ class Annotation(object):
         self.uri, self.modality = uri, modality
         self._tracks = {}
 
+    @staticmethod
+    def _key(key):
+        """(segment, track) from a (segment, track) tuple or a bare Segment (track "_", as pyannote.core)"""
+        if isinstance(key, Segment):
+            return key, DEFAULT_TRACK
+        return key
+
     def __setitem__(self, key, label):
-        segment, track = key
+        segment, track = self._key(key)
         if not isinstance(segment, Segment):
             segment = Segment(*segment)
         if not segment:
@@ -41,7 +66,7 @@ class Annotation(object):
         self._tracks[(segment, track)] = label
 
     def __getitem__(self, key):
-        segment, track = key
+        segment, track = self._key(key)
         if not isinstance(segment, Segment):
             segment = Segment(*segment)
         return self._tracks[(segment, track)]
@@ -79,6 +104,28 @@ class Annotation(object):
 
     def label_tracks(self, label):
         return [(s, t) for s, t, l in self.itertracks(yield_label=True) if l == label]
+
+    def subset(self, labels):
+        """the tracks whose label is in `labels`"""
+        labels = set(labels)
+        out = Annotation(self.uri, self.modality)
+        out._tracks = {k: v for k, v in self._tracks.items() if v in labels}
+        return out
+
+    def smooth(self):
+        """per label, touching or overlapping segments merged into one; tracks renamed A, B, ... label by label"""
+        names = string_generator()
+        out = Annotation(self.uri, self.modality)
+        for label in self.labels():
+            merged = []
+            for segment in sorted(s for (s, _), v in self._tracks.items() if v == label):
+                if merged and segment.start <= merged[-1].end:
+                    merged[-1] = Segment(merged[-1].start, max(merged[-1].end, segment.end))
+                else:
+                    merged.append(segment)
+            for segment in merged:
+                out[segment, next(names)] = label
+        return out
 
     def to_dict(self):
         """{track: label} (track names are unique on this path: one segment per face track)"""

@@ -10,6 +10,9 @@ Mirrors `scripts/pyannote-face.py` of the reference (usage string at :29-89; `tr
   pyannote-face-b200 cluster [--threshold=0.6] <embeddings> <labels> (notebook cells 18-22 as a verb)
   pyannote-face-b200 shot    [--height=50] [--window=2.0] [--threshold=1.0] <video> <output.json>
                              (pyannote-structure.py shot: the <shot.json> that `track` reads)
+  pyannote-face-b200 thread  [--height=200] [--min-match=20] [--lookahead=24] <video> <shot.json> <output.json>
+  pyannote-face-b200 scene   <video> <thread.json> <output.json>
+                             (pyannote-structure.py thread / scene: Annotation JSON of threads, then of scenes)
 
 `docopt`, `ffmpeg` and `pyannote.core` do not exist in the build environment, hence argparse and a
 frame source that reads `.npy` arrays ([T,H,W,3] uint8) or `synthetic:<W>x<H>:<frames>[:<seed>]`;
@@ -80,6 +83,17 @@ class ArrayVideo(object):
                 import cv2
                 rgb = cv2.resize(rgb, self._frame_size)
             yield (i * step, rgb)
+
+    def __call__(self, t):
+        """the frame at time t: index int(frame_rate * t + 1e-5), as the reference Video; IOError outside the clip"""
+        i = int(self.frame_rate * t + 1e-5)
+        if i < 0 or i >= self.frames.shape[0]:
+            raise IOError("no frame at t = %.3f" % t)
+        rgb = np.asarray(self.frames[i])
+        if self._frame_size != self.size:
+            import cv2
+            rgb = cv2.resize(rgb, self._frame_size)
+        return rgb
 
 
 def open_video(spec, frame_rate=25.0):
@@ -227,6 +241,43 @@ def write_timeline(segments, output):
     return content
 
 
+def write_annotation(annotation, output):
+    """-> {"pyannote": "Annotation", "content": [{"segment": {"start", "end"}, "track", "label"}, ...]}"""
+    content = [{"segment": {"start": float(s.start), "end": float(s.end)}, "track": t, "label": l}
+               for s, t, l in annotation.itertracks(yield_label=True)]
+    with open(output, "w") as f:
+        json.dump({"pyannote": "Annotation", "content": content}, f)
+    return content
+
+
+def load_annotation(path):
+    from .annotation import Annotation, Segment
+    with open(path) as f:
+        data = json.load(f)
+    out = Annotation()
+    for item in data["content"] if isinstance(data, dict) else data:
+        out[Segment(float(item["segment"]["start"]), float(item["segment"]["end"])), item["track"]] = item["label"]
+    return out
+
+
+def thread_cmd(video, shot, output, height=200, min_match=20, lookahead=24):
+    """Shot threads (pyannote-structure.py thread) as pyannote.core Annotation JSON"""
+    from .annotation import Segment
+    from .thread import Thread
+    shots = [Segment(s.start, s.end) for s in load_shots(shot)] if isinstance(shot, str) else shot
+    threads = Thread(video, shot=shots, height=height, min_match=min_match, lookahead=lookahead)()
+    write_annotation(threads, output)
+    return threads
+
+
+def scene_cmd(threads, output):
+    """Scenes from threads (Thread.scenes) as pyannote.core Annotation JSON"""
+    from .thread import scenes
+    out = scenes(load_annotation(threads) if isinstance(threads, str) else threads)
+    write_annotation(out, output)
+    return out
+
+
 def cluster_cmd(embeddings, output, threshold=0.6, metric="euclidean"):
     from .clustering import FaceClustering
     clustering = FaceClustering(threshold=threshold, metric=metric)
@@ -284,6 +335,17 @@ def main(argv=None):
     p.add_argument("--height", type=int, default=50)
     p.add_argument("--window", type=float, default=2.0)
     p.add_argument("--threshold", type=float, default=1.0)
+    p = sub.add_parser("thread")
+    p.add_argument("video")
+    p.add_argument("shot")
+    p.add_argument("output")
+    p.add_argument("--height", type=int, default=200)
+    p.add_argument("--min-match", type=int, default=20)
+    p.add_argument("--lookahead", type=int, default=24)
+    p = sub.add_parser("scene")
+    p.add_argument("video")
+    p.add_argument("threads")
+    p.add_argument("output")
     a = ap.parse_args(argv)
     if a.verb == "track":
         track(open_video(a.video, a.frame_rate), a.shot, a.tracking, detect_min_size=a.min_size, detect_every=a.every,
@@ -296,6 +358,11 @@ def main(argv=None):
         detect(open_video(a.video, a.frame_rate), a.detections, detector=a.detector)
     elif a.verb == "shot":
         shot_cmd(open_video(a.video, a.frame_rate), a.output, height=a.height, window=a.window, threshold=a.threshold)
+    elif a.verb == "thread":
+        thread_cmd(open_video(a.video, a.frame_rate), a.shot, a.output, min_match=a.min_match, lookahead=a.lookahead,
+                   height=a.height)
+    elif a.verb == "scene":
+        scene_cmd(a.threads, a.output)
     elif a.verb == "cluster":
         cluster_cmd(a.embeddings, a.labels, threshold=a.threshold, metric=a.metric)
     return 0
